@@ -6,8 +6,9 @@
 
 Default workload (BASELINE.json configs[1], "c2"): vector_quantize_scan, int8 quantized from a synthetic N(0,1) f32
 10M x 384 corpus with the reference's S8 rule, L2 (the default metric), k=20, batch=1.  A "step" is one query scanned against
-the whole resident corpus (3.84 GB >> 126 MB L2, so every step streams from HBM).  The K steps are repeated until the timed
-region lasts >= --min-ms (default 50 ms: at 8 GPUs 20 steps would be a 2 ms sample); `steps_timed` says how many ran.
+the whole resident corpus (3.84 GB >> 126 MB L2, so every step streams from HBM).  Exactly K steps are timed, on queries
+that depend only on the arguments.  `--dump-outputs DIR` writes the top-k the last timed step returned (rowids and distances,
+float64 .npy) so that two builds can be compared output for output.
 
 Our arm prints `value` (queries already in HBM; launch -> candidates -> exact top-k on the host, per query), `e2e` (HOST query
 in, host top-k out through the C ABI call the SQLite plugin makes, vsb_scan_topk, one at a time; the pipelined
@@ -265,6 +266,13 @@ def ncu_fact(pattern: str, key: str):
     return None, None
 
 
+def dump_outputs(dirname: str, arrays: dict):
+    """--dump-outputs: every result array as DIR/<name>.npy in float64 (which holds the int64 rowids exactly)"""
+    os.makedirs(dirname, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(dirname, f"{name}.npy"), np.asarray(arr, dtype=np.float64))
+
+
 # ------------------------------------------------------------------ main
 def main():
     claim_stdout()
@@ -277,7 +285,6 @@ def main():
     ap.add_argument("--n", "--rows", dest="n", type=int, default=0, help="corpus rows (--rows: torchrun's own parser rejects a bare --n as ambiguous)")
     ap.add_argument("--dim", type=int, default=0)
     ap.add_argument("--k", type=int, default=0)
-    ap.add_argument("--min-ms", type=float, default=50.0, help="repeat the K steps until the timed region lasts at least this long")
     ap.add_argument("--cpu-threads", type=int, default=0, help="threads of the CPU reference leg (0 = all cores)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-batched", action="store_true", help="skip the batch=1024 tensor-core legs")
@@ -286,6 +293,7 @@ def main():
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"], help="sharded single queries: NVLink peer-memory push (engine) or NCCL all-gather (round 1)")
     ap.add_argument("--engine-opt", action="append", default=[], help="name=value passed to vsb_set_option (experiments)")
     ap.add_argument("--batch-depth", type=int, default=2, choices=[1, 2], help="sharded batches over the peer exchange: batches in flight")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step to DIR/<name>.npy")
     a = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -421,18 +429,6 @@ def main():
         run_single(0, max(W, 1))
     else:
         run_sharded(0, max(W, 1), True)
-    # how many times the K steps must repeat for the timed region to last >= min_ms (same decision on every rank)
-    barrier()
-    t_probe = time.perf_counter()
-    (run_single if world == 1 else (lambda f, c: run_sharded(f, c, True)))(0, min(K, 4 * G if world > 1 else 16))
-    barrier()
-    est_ms = (time.perf_counter() - t_probe) * 1e3 / min(K, 4 * G if world > 1 else 16)
-    reps = max(1, int(np.ceil(a.min_ms / max(est_ms * K, 1e-6))))
-    if world > 1:
-        t = torch.tensor([reps], device=device)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        reps = int(t.item())
-    KT = K * reps
     if sampler:
         sampler.wait_first(2.0)
     barrier()
@@ -442,7 +438,7 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t_wall0 = time.perf_counter()
     e0.record(st)
-    last, last_qi = run_single(W, KT) if world == 1 else run_sharded(W, KT, True)
+    last, last_qi = run_single(W, K) if world == 1 else run_sharded(W, K, True)
     e1.record(st)
     barrier()
     t_wall = time.perf_counter() - t_wall0
@@ -493,26 +489,26 @@ def main():
         # (a) THE call the SQLite plugin makes from xFilter (vsb_scan_topk), one query at a time: pinned H2D of the query + scan +
         #     filter + D2H of the candidate head + host slot replay, nothing overlapped across queries.  This is e2e.value.
         t0 = time.perf_counter()
-        for i in range(KT):
+        for i in range(K):
             last_e2e = ix.scan_topk(api.L2, q_host[W + (i % (NQ - W - 1))], k)[0]
         e2e_s = time.perf_counter() - t0
-        e2e_qi = W + ((KT - 1) % (NQ - W - 1))
+        e2e_qi = W + ((K - 1) % (NQ - W - 1))
         # (b) the asynchronous pair vsb_scan_submit(host query) / vsb_collect, two queries in flight (what a batching caller gets)
         t0 = time.perf_counter()
         pending = None
-        for i in range(KT):
+        for i in range(K):
             slot = ix.scan_submit(api.L2, q_host[W + (i % (NQ - W - 1))], k, on_device=False, fetch=True)
             if pending is not None:
                 ix.collect(pending, k)
             pending = slot
         ix.collect(pending, k)
-        pipelined_qps = KT / (time.perf_counter() - t0)
+        pipelined_qps = K / (time.perf_counter() - t0)
         avg_surv = (ix.stat("survivors") - surv0) / max(ix.stat("queries") - q0, 1)
     else:
         run_sharded(0, max(W, 1), False)
         barrier()
         t0 = time.perf_counter()
-        last_e2e, e2e_qi = run_sharded(W, KT, False)
+        last_e2e, e2e_qi = run_sharded(W, K, False)
         barrier()
         e2e_s = time.perf_counter() - t0
         t = torch.tensor([e2e_s], device=device)
@@ -614,28 +610,31 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return 0
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"topk_ids": last[0], "topk_distances": last[1],
+                                      "e2e_topk_ids": last_e2e[0], "e2e_topk_distances": last_e2e[1]})
 
     # ---- roofline of the dominant kernel (scan_kernel): algorithmic bytes = rows * dim * 1 B per launch
     pk = peaks()
     shard_bytes = (hi - lo) * dim
-    step_ms = ms_total / KT
+    step_ms = ms_total / K
     achieved = shard_bytes / (step_ms * 1e-3) / 1e9
     traffic, traffic_src = (ncu_fact("scan_kernel_traffic", "dram_bytes_per_launch") if (world == 1 and n == 10_000_000 and dim == 384) else (None, None))
 
     out = {
-        "metric": METRIC_NAME, "value": KT / (ms_total * 1e-3), "unit": "queries/s", "n_gpus": world, "steps": K, "warmup": W,
-        "steps_timed": KT, "ms_per_step": step_ms, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "int8",
+        "metric": METRIC_NAME, "value": K / (ms_total * 1e-3), "unit": "queries/s", "n_gpus": world, "steps": K, "warmup": W,
+        "steps_timed": K, "ms_per_step": step_ms, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "int8",
         "data": "synthetic N(0,1) f32 (seed 1234) quantized to int8 with the reference S8 rule; queries seed 4321",
         "config": {"workload": workload, "metric": "L2", "k": k, "batch": 1, "rows": n, "dim": dim, "shards": world,
                    "l2_flush": "none needed: each step streams the whole shard (%.2f GB) which exceeds the 126 MB L2" % (shard_bytes / 1e9),
                    "result_mode": "exact reference slot replay (bit-exact rowids/order/distances vs distance-cpu.c)",
-                   "timed_region": f"the {K} steps repeated {reps}x back to back so that the region lasts >= {a.min_ms:.0f} ms",
+                   "timed_region": f"the {K} steps back to back",
                    "in_flight": 2 if world == 1 else depth * G,
                    "exchange": None if world == 1 else (
                        f"groups of {G} independent queries, {depth} groups in flight; every filter kernel stores its result head into every peer's gather buffer over NVLink "
                        "(cudaIpc peer memory) and raises a flag; the receiver waits on the flags on its own stream, one D2H per group, host slot replay (no collective library on the data path)"
                        if a.exchange == "peer" else f"groups of {G} queries: one NCCL all-gather of the shards' result heads + one D2H per group")},
-        "e2e": {"value": KT / e2e_s, "unit": "queries/s", "h2d_bytes_per_step": int(pitch),
+        "e2e": {"value": K / e2e_s, "unit": "queries/s", "h2d_bytes_per_step": int(pitch),
                 "d2h_bytes_per_step": d2h_bytes, "avg_candidates_per_query": avg_surv, "pipelined_value": pipelined_qps,
                 "note": ("value = the synchronous vsb_scan_topk call the SQLite plugin makes from xFilter, one query at a time (pinned H2D of the query, scan + filter kernels, "
                          "one D2H of the candidate head, host slot replay); pipelined_value = vsb_scan_submit(host query)/vsb_collect with two queries in flight"
@@ -643,7 +642,7 @@ def main():
                          "vsb_exchange_submit with HOST queries (pinned H2D per query) + scan/filter kernels on every rank + peer-memory push of the heads + D2H + host slot replay, same grouping as value")},
         "gpu_launches": int(launches),
         "roofline": {"bound": "hbm", "achieved": achieved, "peak": pk["hbm"], "unit": "GB/s", "frac": achieved / pk["hbm"], "traffic": traffic,
-                     "traffic_source": traffic_src, "kernel": "vsb::scan_kernel<int8,L2>", "avg_launch_ms": step_ms, "launches_timed": KT,
+                     "traffic_source": traffic_src, "kernel": "vsb::scan_kernel<int8,L2>", "avg_launch_ms": step_ms, "launches_timed": K,
                      "kernel_alone_ms": alone_ms, "kernel_alone_gbs": (shard_bytes / (alone_ms * 1e-3) / 1e9) if alone_ms else None,
                      "filter_kernel_alone_ms": filter_ms, "peak_source": pk["source"] + " hbm_gbs",
                      "algorithmic_bytes_per_launch": int(shard_bytes),
@@ -885,7 +884,7 @@ def run_c4(torch, a, rank, local_rank, world):
     import sqlite_vector_b200 as vs
     from sqlite_vector_b200 import api, shard
     n, dim, k, B = a.n or 50_000_000, a.dim or 1536, a.k or 100, 256
-    K, W = max(min(a.steps, 20), 1), max(a.warmup, 1)
+    K, W = max(a.steps, 1), max(a.warmup, 1)
     torch.cuda.set_device(local_rank)
     device = torch.device("cuda", local_rank)
     if world > 1:
@@ -978,6 +977,8 @@ def run_c4(torch, a, rank, local_rank, world):
         if world > 1:
             dist.destroy_process_group()
         return 0
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"topk_ids": rb[0], "topk_distances": rb[1], "topk_counts": rb[2]})
     pk = peaks()
     int8_peak, int8_note = measure_int8_peak(torch, device)
     ops = 2.0 * B * tc_rows * dim

@@ -198,10 +198,6 @@ class RefHarness:
                                                 _ptr(q.view(np.uint8).reshape(-1)), qbytes, threads, reps, C.byref(cs)))
 
 
-def have_ref() -> bool:
-    return os.path.exists(os.path.join(REF_DIR, "libref_cpu.so"))
-
-
 # ---------------------------------------------------------------- deterministic inputs (SURVEY §8d)
 def gen_f32(n: int, dim: int, seed: int) -> np.ndarray:
     return np.random.Generator(np.random.PCG64(seed)).standard_normal((n, dim), dtype=np.float32)

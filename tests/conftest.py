@@ -9,7 +9,7 @@ if ROOT not in sys.path:
 
 
 def pytest_configure(config):
-    config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box via gpurun)")
+    config.addinivalue_line("markers", "gpu: needs a CUDA device")
 
 
 @pytest.fixture(scope="session")
@@ -20,15 +20,11 @@ def oracle():
 
 @pytest.fixture(scope="session")
 def ref_cpu():
-    from oracle import pyoracle
-    if not pyoracle.have_ref():
-        pytest.skip("oracle/_ref not built (reference tree absent)")
-    return pyoracle.RefHarness("cpu")
+    from tests import refgolden
+    return refgolden.Reference("cpu")
 
 
 @pytest.fixture(scope="session")
 def ref_avx2():
-    from oracle import pyoracle
-    if not pyoracle.have_ref():
-        pytest.skip("oracle/_ref not built (reference tree absent)")
-    return pyoracle.RefHarness("avx2")
+    from tests import refgolden
+    return refgolden.Reference("avx2")

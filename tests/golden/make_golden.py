@@ -1,7 +1,9 @@
 """Generate tests/golden/*.npz from the UNMODIFIED reference (oracle/_ref, built by oracle/Makefile
-from /root/reference).  Run here (the reference tree is not on the GPU box):
+from the reference tree):
 
-    make -C oracle && python tests/golden/make_golden.py
+    make -C oracle REF=<reference tree> && python tests/golden/make_golden.py
+    python tests/golden/make_golden.py --record          # reference answers replayed by tests/refgolden.py
+    python tests/golden/make_golden.py --abi <dir of sqlite3ext.h>
 
 Everything written is produced by reference code: distances by dispatch_distance_table (stock "CPU"
 build = distance-cpu.c), quantized bytes by quantize_*, top-k by vQuantRunMemory / the vFullScanRun
@@ -90,7 +92,7 @@ def main():
         print(f, os.path.getsize(os.path.join(OUT, f)), "bytes")
 
 
-if __name__ == "__main__" and "--sql" not in sys.argv and "--c1" not in sys.argv:
+if __name__ == "__main__" and not {"--sql", "--c1", "--record", "--abi"} & set(sys.argv):
     main()
 
 
@@ -124,3 +126,49 @@ def c1_golden():
 
 if __name__ == "__main__" and "--c1" in sys.argv:
     c1_golden()
+
+
+RECORDED_TESTS = ["tests/test_oracle_vs_reference.py", "tests/test_oracle_fuzz.py", "tests/test_sql_fuzz.py",
+                  "tests/test_sql_surface.py::test_surface_matches_live_reference"]
+
+
+def record():
+    """run the tests that compare with the reference against its live build, and store every answer it gave them"""
+    import pytest
+    from tests import refgolden
+    refgolden.RECORDING = True
+    rc = pytest.main(["-q", "-p", "no:cacheprovider", "-m", "not gpu"] + [os.path.join(ROOT, t) for t in RECORDED_TESTS])
+    if rc != 0:
+        raise SystemExit(f"pytest exited with {rc}: nothing recorded")
+    refgolden.save()
+    for f in (refgolden.CALLS, refgolden.SQL):
+        print(os.path.relpath(f, ROOT), os.path.getsize(f), "bytes")
+
+
+if __name__ == "__main__" and "--record" in sys.argv:
+    record()
+
+
+def abi_slots(hdr_dir):
+    """slot of every sqlite3_api_routines member, as the compiler lays the struct out: offsetof / sizeof(void *)"""
+    import json
+    import subprocess
+    import tempfile
+    sys.path.insert(0, os.path.join(ROOT, "tools"))
+    from gen_sqlite_abi import members
+    names = members(os.path.join(hdr_dir, "sqlite3ext.h"))
+    lines = "\n".join(f'    printf("%s %zu\\n", "{n}", offsetof(sqlite3_api_routines, {n}) / sizeof(void *));' for n in names)
+    src = "#include <stddef.h>\n#include <stdio.h>\n#include \"sqlite3ext.h\"\nint main(void) {\n" + lines + "\n    return 0;\n}\n"
+    with tempfile.TemporaryDirectory() as tmp:
+        with open(os.path.join(tmp, "slots.c"), "w") as f:
+            f.write(src)
+        subprocess.run(["gcc", "-I", hdr_dir, "-o", os.path.join(tmp, "slots"), os.path.join(tmp, "slots.c")], check=True)
+        out = subprocess.run([os.path.join(tmp, "slots")], capture_output=True, text=True, check=True).stdout
+    slots = {n: int(i) for n, i in (ln.split() for ln in out.splitlines())}
+    with open(os.path.join(OUT, "sqlite3_api_slots.json"), "w") as f:
+        json.dump(slots, f, indent=0)
+    print("sqlite3_api_slots.json:", len(slots), "members")
+
+
+if __name__ == "__main__" and "--abi" in sys.argv:
+    abi_slots(sys.argv[sys.argv.index("--abi") + 1])

@@ -1,7 +1,7 @@
 """Pins oracle/vs_oracle.c against the UNMODIFIED reference (oracle/_ref, built by oracle/Makefile).
 
-Runs only where the reference tree was available to build oracle/_ref (this container); the
-committed fixtures in tests/golden/ carry the same evidence to machines without it.
+The reference's answers to these calls are recorded once from that build (tests/refgolden.py), so the
+comparison runs on machines without the reference sources.
 """
 import numpy as np
 import pytest

@@ -1,20 +1,18 @@
-"""Differential tests of the host side of the SQL surface against the LIVE reference extension (oracle/_ref/cpu/vector.so), each
-in its own process: the vector_as_* encoders on drawn JSON / BLOB inputs (number formats, separators, brackets, dimension
-arguments) and vector_quantize builds on drawn tables (5 source types, dims 1..40, NULL rows, NaN / Inf / huge values, constant
-and non-negative columns, both qtypes, several max_memory settings) — rows, error strings, shadow-table bytes and metadata
-must be identical.  CPU only (without a GPU vector_quantize runs its host loops; the GPU loops are pinned to the same bytes by
+"""Differential tests of the host side of the SQL surface against the reference extension (its stock build; answers recorded by
+tests/refgolden.py), each script in its own process: the vector_as_* encoders on drawn JSON / BLOB inputs (number formats,
+separators, brackets, dimension arguments) and vector_quantize builds on drawn tables (5 source types, dims 1..40, NULL rows,
+NaN / Inf / huge values, constant and non-negative columns, both qtypes, several max_memory settings) — rows, error strings,
+shadow-table bytes and metadata must be identical.  CPU only (without a GPU vector_quantize runs its host loops; the GPU loops are pinned to the same bytes by
 test_gpu_parity.py / test_sql_surface.py).  Seeds are fixed; 24 000 encoder statements and 240 table scripts were run once
 offline without a mismatch."""
-import os
 import random
 
 import numpy as np
 import pytest
 
 from oracle import pyoracle as po
-from tests.sqlrun import OURS, REF_CPU, blob, run_sql
-
-needs_ref = pytest.mark.skipif(not os.path.exists(REF_CPU + ".so"), reason="oracle/_ref not built (reference tree absent)")
+from tests.refgolden import run_reference_sql
+from tests.sqlrun import OURS, blob, run_sql
 
 NUMS = ["0", "1", "-1", "2.5", "-3e2", "1e-7", "+5", ".5", "5.", "1e400", "-1e400", "1e-400", "nan", "NaN", "inf", "-inf", "Infinity", "0x10", "1_000", "",
         "--1", "1e", "1e+", "127", "-128", "128", "-129", "255", "256", "3.9", "-3.9", "65504", "65520", "70000", "1e38", "3.5e38", "0.1", "1e-45", "007", "1.0.0",
@@ -63,12 +61,11 @@ def _encoder_stmt(rng):
     return f"SELECT hex({f}({arg}, {rng.choice(['0', '1', '2', '3', '4', '5', '8', '-1', 'NULL', chr(39) + '3' + chr(39), '2.0', '1000000'])}))"
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", [3, 17])
 def test_encoders_match_live_reference(seed):
     rng = random.Random(seed)
     script = [_encoder_stmt(rng) for _ in range(400)]
-    ours, ref = run_sql(OURS, script), run_sql(REF_CPU, script)
+    ours, ref = run_sql(OURS, script), run_reference_sql(script)
     for s, a, b in zip(script, ours, ref):
         assert a == b, (s, a, b)
 
@@ -112,11 +109,10 @@ def _quantize_script(seed):
     return s
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", [1, 2, 5, 8, 13, 21])
 def test_quantize_builds_match_live_reference(seed):
     script = _quantize_script(seed)
-    ours, ref = run_sql(OURS, script, env={"CUDA_VISIBLE_DEVICES": ""}), run_sql(REF_CPU, script)
+    ours, ref = run_sql(OURS, script, env={"CUDA_VISIBLE_DEVICES": ""}), run_reference_sql(script)
     for s, a, b in zip(script, ours, ref):
         assert a == b, (s if isinstance(s, str) else s[0], str(a)[:300], str(b)[:300])
 
@@ -145,7 +141,6 @@ def _option_string(rng):
     return s
 
 
-@needs_ref
 @pytest.mark.parametrize("block", [0, 1])
 def test_option_strings_match_live_reference(block):
     """vector_init / vector_quantize option strings (the key=value parser, unknown keys, bad values): same rows, same error
@@ -165,7 +160,7 @@ def test_option_strings_match_live_reference(block):
                   f"SELECT vector_quantize('o', 'e', '{_option_string(rng)}')",
                   "SELECT key, value FROM _sqliteai_vector WHERE tblname='o' ORDER BY key",
                   "SELECT count(*), sum(length(data)) FROM vector0_o_e"]
-        ours, ref = run_sql(OURS, script, env={"CUDA_VISIBLE_DEVICES": ""}), run_sql(REF_CPU, script)
+        ours, ref = run_sql(OURS, script, env={"CUDA_VISIBLE_DEVICES": ""}), run_reference_sql(script)
         quantize_failed = ours[5] == ref[5] and ("error" in ours[5] or ours[5]["rows"] == [[None]])     # error, or the silent NULL of a rejected option string
         for i, (s, a, b) in enumerate(zip(script, ours, ref)):
             if i == 7 and quantize_failed:
