@@ -111,14 +111,12 @@ constexpr int kSlots = 32;               // result slots: queries in flight (the
                                          // kSlots / 2 queries in flight so that a peer never overwrites a gather row that is still being read)
 
 // result block of one query, written by filter_kernel into DEVICE memory and fetched with one async copy:
-//   head = [hdr: 16 ints][table: kTableCap x int2][first kFirstFetch survivors x uint2]   (kHeadBytes, what travels)
+//   head = the result head (layout in scan_kernels.cuh) with room for the first kFirstFetch survivors (kHeadBytes, what travels)
 //   tail = the (rare) survivors beyond kFirstFetch, fetched by a second copy.
 // The heads of all slots are ONE contiguous allocation (slot s at s * kHeadBytes), so a launcher can all-gather the
 // heads of a group of consecutive slots with a single collective.  (Zero-copy writes of ~300 scattered 8-byte records
 // over PCIe made the filter kernel 5x slower than writing to HBM and copying once.)
-constexpr int kTableCap = 512;
 constexpr int kFirstFetch = 1024;
-constexpr size_t kResHdrBytes = 64 + sizeof(int2) * kTableCap;
 constexpr size_t kHeadBytes = kResHdrBytes + sizeof(uint2) * kFirstFetch;
 
 // scan workspace of ONE query (per-stream k-lists / CTA lists, in-CTA bounds, candidate logs): written by scan_kernel,
@@ -143,15 +141,14 @@ constexpr int kWorks = 4;
 
 struct Slot {
     uint8_t *d_res = nullptr, *h_res = nullptr;      // this slot's head inside vsb_index::d_heads / h_heads
-    uint2 *h_out = nullptr, *d_out = nullptr;        // first kFirstFetch survivors (inside the head)
+    uint2 *d_out = nullptr;                          // first kFirstFetch survivors (inside the head)
     uint2 *h_tail = nullptr, *d_tail = nullptr;      // survivors kFirstFetch.. (inside vsb_index::d_tails / h_tails)
-    int2 *h_table = nullptr, *d_table = nullptr;
-    int *h_hdr = nullptr, *d_hdr = nullptr;
+    int2 *d_table = nullptr;
+    int *d_hdr = nullptr;
     uint8_t *h_query = nullptr, *d_query = nullptr;  // pinned staging + device copy of the query
     int *d_ctrl = nullptr;
     cudaEvent_t done = nullptr;   // recorded after the result block of this slot has been copied to the host
     int seq = 0;
-    int nblocks = 0;
 };
 
 }  // namespace
@@ -254,7 +251,7 @@ Plan make_plan(const vsb_index *ix, int kcap) {
     size_t avail = (size_t)ix->max_smem > fixed ? (size_t)ix->max_smem - fixed : 0;
     if (g_opt_ring_bytes > 0 && (size_t)g_opt_ring_bytes < avail) avail = (size_t)g_opt_ring_bytes;
     const size_t wtile = (size_t)(32 >> log2P) * pitch;
-    // leave room on the SM for one filter block of the previous query (it runs beside the scan CTA, see launch_scan)
+    // leave room on the SM for one filter block of the previous query (it runs beside the scan CTA, see launch_scan_group)
     const size_t reserve = filter_fast_smem(ix->num_sms) + 3072;
     if (kcap > 0 && kcap <= 32 && avail > reserve && (avail - reserve) / kWarps / (wtile ? wtile : 1) >= 2) avail -= reserve;
     int nsw = (int)(avail / kWarps / (wtile ? wtile : 1));
@@ -314,9 +311,9 @@ int ensure_slots_alloc(vsb_index *ix) {
         s.h_res = ix->h_heads + kHeadBytes * i;
         s.d_tail = (uint2 *)(ix->d_tails + tail_bytes * i);
         s.h_tail = (uint2 *)(ix->h_tails + tail_bytes * i);
-        s.d_hdr = (int *)s.d_res; s.h_hdr = (int *)s.h_res;
-        s.d_table = (int2 *)(s.d_res + 64); s.h_table = (int2 *)(s.h_res + 64);
-        s.d_out = (uint2 *)(s.d_res + kResHdrBytes); s.h_out = (uint2 *)(s.h_res + kResHdrBytes);
+        s.d_hdr = (int *)s.d_res;
+        s.d_table = (int2 *)(s.d_res + kHdrBytes);
+        s.d_out = (uint2 *)(s.d_res + kResHdrBytes);
         s.h_query = hq + (size_t)ix->pitch * i;
         s.d_query = dq + (size_t)ix->pitch * i;
         s.d_ctrl = dc + 4 * i;
@@ -333,6 +330,21 @@ int ensure_slots(vsb_index *ix) {
     return VSB_OK;
 }
 
+// the device buffers of all scan workspaces (their events stay)
+void free_workspaces(vsb_index *ix) {
+    ix->ws_kcap = 0;
+    for (Work &w : ix->work) {
+        for (QWork &q : w.q) {
+            cudaFree(q.d_lists); cudaFree(q.d_logs); cudaFree(q.d_counts); cudaFree(q.d_tlocal);
+            q = QWork();
+        }
+        cudaFree(w.d_bounds); cudaFree(w.d_cta_time);
+        w.d_bounds = nullptr; w.d_cta_time = nullptr;
+        w.bounds_tiles = -1;
+        w.in_use = false;
+    }
+}
+
 int ensure_workspace(vsb_index *ix, int k) {
     const int kcap = (k + 31) & ~31;
     const int logcap = std::max(256, 12 * k);
@@ -341,26 +353,14 @@ int ensure_workspace(vsb_index *ix, int k) {
     CU(cudaStreamSynchronize(ix->stream));       // queries in flight still use the old workspaces
     CU(cudaStreamSynchronize(ix->stream2));
     CU(cudaStreamSynchronize(ix->fstream));
-    ix->ws_kcap = 0;
-    for (int i = 0; i < kWorks; ++i) {
-        Work &w = ix->work[i];
-        for (int g = 0; g < kMaxGroup; ++g) {
-            QWork &q = w.q[g];
-            if (q.d_lists) cudaFree(q.d_lists);
-            if (q.d_logs) cudaFree(q.d_logs);
-            if (q.d_counts) cudaFree(q.d_counts);
-            if (q.d_tlocal) cudaFree(q.d_tlocal);
-            q.d_lists = nullptr; q.d_logs = nullptr; q.d_counts = nullptr; q.d_tlocal = nullptr;
+    free_workspaces(ix);
+    for (Work &w : ix->work) {
+        for (QWork &q : w.q) {
             CU(cudaMalloc((void **)&q.d_lists, sizeof(float) * (size_t)streams * kcap));
             CU(cudaMalloc((void **)&q.d_logs, sizeof(uint2) * (size_t)streams * logcap));
             CU(cudaMalloc((void **)&q.d_counts, sizeof(int) * (size_t)streams));
             CU(cudaMalloc((void **)&q.d_tlocal, sizeof(float) * (size_t)streams));
         }
-        if (w.d_bounds) cudaFree(w.d_bounds);
-        if (w.d_cta_time) cudaFree(w.d_cta_time);
-        w.d_bounds = nullptr; w.d_cta_time = nullptr;
-        w.bounds_tiles = -1;
-        w.in_use = false;
         CU(cudaMalloc((void **)&w.d_bounds, sizeof(long long) * (size_t)(ix->num_sms + 1)));
         CU(cudaMalloc((void **)&w.d_cta_time, sizeof(unsigned) * (size_t)ix->num_sms));
         if (!w.scanned) CU(cudaEventCreateWithFlags(&w.scanned, cudaEventDisableTiming));
@@ -499,7 +499,6 @@ int launch_scan_group(vsb_index *ix, int metric, const uint8_t *const *d_queries
             q.seqno = ++slot->seq;
             q.xslot = (int)(slot - ix->slot);
             q.xseq = push ? exchange_next_seq(ix, q.xslot) : 0u;
-            slot->nblocks = nblocks;
         }
         f.bounds = balance ? wk->d_bounds : nullptr;
         f.cta_time = wk->d_cta_time;
@@ -532,10 +531,6 @@ int launch_scan_group(vsb_index *ix, int metric, const uint8_t *const *d_queries
     return VSB_OK;
 }
 
-int launch_scan(vsb_index *ix, int metric, const uint8_t *d_query, int k, Slot *slot, float *d_dist_all, bool fetch, cudaStream_t ss) {
-    return launch_scan_group(ix, metric, &d_query, 1, k, slot ? &slot : nullptr, d_dist_all, fetch, ss);
-}
-
 // single-query scans alternate between two streams (option scan_streams, see g_opt_scan_streams)
 cudaStream_t next_scan_stream(vsb_index *ix) {
     if (g_opt_scan_streams < 2) return ix->stream;
@@ -548,84 +543,94 @@ inline int64_t rowid_of(const vsb_index *ix, uint32_t local) {
 }
 
 // ------------------------------------------------------------------ the reference's k-slot algorithm
-struct SlotState {
-    int k, mi;
-    double *dist;
-    int64_t *ids;
-};
 inline int first_max(const double *v, int n) {  // first index of the maximum, strict '>' (:2022-2049)
     int b = 0;
     for (int i = 1; i < n; ++i)
         if (v[i] > v[b]) b = i;
     return b;
 }
-inline void slots_begin(SlotState &s) {  // :1808-1813 (max_index is carried over, not reset)
-    for (int i = 0; i < s.k; ++i) { s.dist[i] = std::numeric_limits<double>::infinity(); s.ids[i] = 0; }
-    if (s.mi < 0 || s.mi >= s.k) s.mi = 0;
-}
-inline void slots_offer(SlotState &s, float d, int64_t id) {  // :2102-2106 / :2145-2152
-    if ((double)d < s.dist[s.mi]) {
-        s.dist[s.mi] = (double)d;
-        s.ids[s.mi] = id;
-        s.mi = first_max(s.dist, s.k);
+// the k slots of one query: started with the max_index carried over from the previous query, offered the candidates in scan
+// order, finished into the sorted result
+struct SlotReplay {
+    int k, mi;
+    double *dist;
+    int64_t *ids;
+    SlotReplay(int k_, int max_index, double *dist_, int64_t *ids_) : k(k_), mi(max_index), dist(dist_), ids(ids_) {   // :1808-1813
+        for (int i = 0; i < k; ++i) { dist[i] = std::numeric_limits<double>::infinity(); ids[i] = 0; }
+        if (mi < 0 || mi >= k) mi = 0;
     }
-}
-inline int slots_finish(SlotState &s) {  // exchange sort + INF trim (:2051-2069, :1816-1817)
-    const double inf = std::numeric_limits<double>::infinity();
-    int unused = 0;
-    for (int i = 0; i + 1 < s.k; ++i) {
-        if (s.dist[i] == inf) ++unused;
-        for (int j = i + 1; j < s.k; ++j)
-            if (s.dist[j] < s.dist[i]) { std::swap(s.dist[i], s.dist[j]); std::swap(s.ids[i], s.ids[j]); }
+    void offer(float d, int64_t id) {  // :2102-2106 / :2145-2152
+        if ((double)d < dist[mi]) {
+            dist[mi] = (double)d;
+            ids[mi] = id;
+            mi = first_max(dist, k);
+        }
     }
-    if (s.dist[s.k - 1] == inf) ++unused;
-    return s.k - unused;
+    void offer_bits(uint32_t bits, int64_t id) {   // a candidate's distance as the GPU stored it
+        float d;
+        memcpy(&d, &bits, 4);
+        offer(d, id);
+    }
+    int finish() {  // exchange sort + INF trim (:2051-2069, :1816-1817); returns the used slots
+        const double inf = std::numeric_limits<double>::infinity();
+        int unused = 0;
+        for (int i = 0; i + 1 < k; ++i) {
+            if (dist[i] == inf) ++unused;
+            for (int j = i + 1; j < k; ++j)
+                if (dist[j] < dist[i]) { std::swap(dist[i], dist[j]); std::swap(ids[i], ids[j]); }
+        }
+        if (dist[k - 1] == inf) ++unused;
+        return k - unused;
+    }
+};
+
+// ------------------------------------------------------------------ result heads on the host (layout in scan_kernels.cuh)
+// survivors that a head carries itself (a head whose kHdrHeadcap is unset or out of range: kFirstFetch)
+inline int head_cap(const int *hdr) {
+    const int c = hdr[kHdrHeadcap];
+    return (c > 0 && c <= kFirstFetch) ? c : kFirstFetch;
+}
+
+// walks the survivors of a result head in scan order: visit(distance bits, local row).  Survivors beyond the head's headcap
+// are read from tail (nullptr when the head holds them all).  Returns how many were visited.
+template <class Visit>
+int visit_head(const uint8_t *head, const uint2 *tail, Visit visit) {
+    const int *hdr = (const int *)head;
+    const int2 *table = (const int2 *)(head + kHdrBytes);
+    const uint2 *out = (const uint2 *)(head + kResHdrBytes);
+    const int headcap = head_cap(hdr), nblocks = hdr[kHdrBlocks];
+    int n = 0;
+    for (int b = 0; b < nblocks; ++b) {
+        const int2 t = table[b];
+        for (int i = 0; i < t.y; ++i, ++n) {
+            const int at = t.x + i;
+            const uint2 c = at < headcap ? out[at] : tail[at - headcap];
+            visit(c.x, c.y);
+        }
+    }
+    return n;
 }
 
 // gather the survivors of a finished slot in scan order; returns count or <0
 int gather_survivors(vsb_index *ix, Slot *slot, std::vector<uint2> &out, bool *overflow) {
     *overflow = false;
-    if (slot->h_hdr[2] != slot->seq) return fail(VSB_ECUDA, "scan result header not published (seq %d != %d)", slot->h_hdr[2], slot->seq);
-    if (slot->h_hdr[1]) { *overflow = true; return 0; }
-    const int total = slot->h_hdr[0];
-    if (total > kFirstFetch) {  // rare: fetch the tail of the survivor list
-        if (cudaMemcpyAsync(slot->h_tail, slot->d_tail, sizeof(uint2) * (size_t)(total - kFirstFetch),
+    const int *hdr = (const int *)slot->h_res;
+    if (hdr[kHdrSeq] != slot->seq) return fail(VSB_ECUDA, "scan result header not published (seq %d != %d)", hdr[kHdrSeq], slot->seq);
+    if (hdr[kHdrFlags]) { *overflow = true; return 0; }
+    const int total = hdr[kHdrTotal], headcap = head_cap(hdr);
+    if (total > headcap) {  // rare: fetch the tail of the survivor list
+        if (cudaMemcpyAsync(slot->h_tail, slot->d_tail, sizeof(uint2) * (size_t)(total - headcap),
                             cudaMemcpyDeviceToHost, ix->fstream) != cudaSuccess ||
             cudaStreamSynchronize(ix->fstream) != cudaSuccess)
             return fail(VSB_ECUDA, "fetching %d survivors failed: %s", total, cudaGetErrorString(cudaGetLastError()));
     }
     out.clear();
     out.reserve((size_t)total);
-    for (int b = 0; b < slot->nblocks; ++b) {
-        const int2 t = slot->h_table[b];
-        for (int i = 0; i < t.y; ++i) {
-            const int at = t.x + i;
-            out.push_back(at < kFirstFetch ? slot->h_out[at] : slot->h_tail[at - kFirstFetch]);
-        }
-    }
+    const int n = visit_head(slot->h_res, slot->h_tail, [&](uint32_t bits, uint32_t row) { out.push_back(make_uint2(bits, row)); });
     ix->st_queries++;
-    ix->st_survivors += (long long)out.size();
-    ix->st_last_survivors = (long long)out.size();
-    return (int)out.size();
-}
-
-int streamed_scan_all(vsb_index *ix, int metric, const uint8_t *d_query, float *out_dist);
-
-int scan_all_into(vsb_index *ix, int metric, const uint8_t *d_query, std::vector<float> &dist) {
-    if (ix->streamed) {
-        dist.resize((size_t)ix->n);
-        return streamed_scan_all(ix, metric, d_query, dist.data());
-    }
-    if (!ix->d_dist_all) {
-        CU(cudaMalloc((void **)&ix->d_dist_all, sizeof(float) * (size_t)std::max<long long>(ix->cap, 1)));
-        ix->dev_bytes += sizeof(float) * (size_t)ix->cap;
-    }
-    int rc = launch_scan(ix, metric, d_query, 0, nullptr, ix->d_dist_all, true, ix->stream);
-    if (rc) return rc;
-    dist.resize((size_t)ix->n);
-    CU(cudaMemcpyAsync(dist.data(), ix->d_dist_all, sizeof(float) * (size_t)ix->n, cudaMemcpyDeviceToHost, ix->stream));
-    CU(cudaStreamSynchronize(ix->stream));
-    return VSB_OK;
+    ix->st_survivors += n;
+    ix->st_last_survivors = n;
+    return n;
 }
 
 int stage_query(vsb_index *ix, Slot *slot, const void *query, cudaStream_t ss) {
@@ -710,57 +715,63 @@ int streamed_candidates(vsb_index *ix, int metric, const uint8_t *d_query, int k
         });
 }
 
+// the all-distances path (k > kMaxK, a candidate overflow, vsb_scan_all): stages a host query on slot 0 and computes the
+// distance of every row, resident or streamed, into dist (scan order)
+int query_all_distances(vsb_index *ix, int metric, const void *query, std::vector<float> &dist) {
+    CU(cudaSetDevice(ix->device));
+    int rc = ensure_slots(ix);
+    if (rc) return rc;
+    rc = stage_query(ix, &ix->slot[0], query, ix->stream);
+    if (rc) return rc;
+    const uint8_t *d_query = ix->slot[0].d_query;
+    dist.resize((size_t)ix->n);
+    if (ix->streamed) return streamed_scan_all(ix, metric, d_query, dist.data());
+    if (!ix->d_dist_all) {
+        CU(cudaMalloc((void **)&ix->d_dist_all, sizeof(float) * (size_t)std::max<long long>(ix->cap, 1)));
+        ix->dev_bytes += sizeof(float) * (size_t)ix->cap;
+    }
+    rc = launch_scan_group(ix, metric, &d_query, 1, 0, nullptr, ix->d_dist_all, true, ix->stream);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(dist.data(), ix->d_dist_all, sizeof(float) * (size_t)ix->n, cudaMemcpyDeviceToHost, ix->stream));
+    CU(cudaStreamSynchronize(ix->stream));
+    return VSB_OK;
+}
+
 // one query, host in / candidates out (sorted by scan order).  Falls back to the all-distances kernel when the
 // candidate log overflowed or k is larger than the candidate path supports (still GPU-computed distances).
 int query_candidates(vsb_index *ix, int metric, const void *query, int k, std::vector<uint2> &cands) {
     CU(cudaSetDevice(ix->device));
     int rc = ensure_slots(ix);
     if (rc) return rc;
-    Slot *slot = &ix->slot[ix->streamed ? kSlots - 1 : 0];   // streamed: slots 0..3 rotate over the windows, the query is parked in the last one
-    rc = stage_query(ix, slot, query, ix->stream);   // synchronous call: one stream (a possible all-distances fallback reads d_query on it)
-    if (rc) return rc;
     bool overflow = (k > kMaxK);
-    if (ix->streamed) {
-        if (!overflow) {
-            rc = ensure_workspace(ix, k);
-            if (rc) return rc;
-            rc = streamed_candidates(ix, metric, slot->d_query, k, cands, &overflow);
-            if (rc) return rc;
-        }
-        if (overflow) {
-            ix->st_fallbacks++;
-            std::vector<float> dist;
-            rc = scan_all_into(ix, metric, slot->d_query, dist);
-            if (rc) return rc;
-            cands.resize((size_t)ix->n);
-            for (long long i = 0; i < ix->n; ++i) {
-                uint32_t bits;
-                memcpy(&bits, &dist[(size_t)i], 4);
-                cands[(size_t)i] = make_uint2(bits, (uint32_t)i);
-            }
-        }
-        return VSB_OK;
-    }
     if (!overflow) {
+        Slot *slot = &ix->slot[ix->streamed ? kSlots - 1 : 0];   // streamed: slots 0..3 rotate over the windows, the query is parked in the last one
+        rc = stage_query(ix, slot, query, ix->stream);
+        if (rc) return rc;
         rc = ensure_workspace(ix, k);
         if (rc) return rc;
-        rc = launch_scan(ix, metric, slot->d_query, k, slot, nullptr, true, ix->stream);
-        if (rc) return rc;
-        CU(cudaEventSynchronize(slot->done));
-        int n = gather_survivors(ix, slot, cands, &overflow);
-        if (n < 0) return n;
-    }
-    if (overflow) {
-        ix->st_fallbacks++;
-        std::vector<float> dist;
-        rc = scan_all_into(ix, metric, slot->d_query, dist);
-        if (rc) return rc;
-        cands.resize((size_t)ix->n);
-        for (long long i = 0; i < ix->n; ++i) {
-            uint32_t bits;
-            memcpy(&bits, &dist[(size_t)i], 4);
-            cands[(size_t)i] = make_uint2(bits, (uint32_t)i);
+        if (ix->streamed) {
+            rc = streamed_candidates(ix, metric, slot->d_query, k, cands, &overflow);
+            if (rc) return rc;
+        } else {
+            const uint8_t *dq = slot->d_query;
+            rc = launch_scan_group(ix, metric, &dq, 1, k, &slot, nullptr, true, ix->stream);
+            if (rc) return rc;
+            CU(cudaEventSynchronize(slot->done));
+            const int n = gather_survivors(ix, slot, cands, &overflow);
+            if (n < 0) return n;
         }
+    }
+    if (!overflow) return VSB_OK;
+    ix->st_fallbacks++;
+    std::vector<float> dist;
+    rc = query_all_distances(ix, metric, query, dist);
+    if (rc) return rc;
+    cands.resize((size_t)ix->n);
+    for (long long i = 0; i < ix->n; ++i) {
+        uint32_t bits;
+        memcpy(&bits, &dist[(size_t)i], 4);
+        cands[(size_t)i] = make_uint2(bits, (uint32_t)i);
     }
     return VSB_OK;
 }
@@ -953,6 +964,14 @@ static int stage_acquire(vsb_index *ix, int *which) {
     return VSB_OK;
 }
 
+// switches ix from implicit rowids (first_seq + row + 1) to an explicit list, filled in for the rows appended so far
+static void materialise_ids(vsb_index *ix) {
+    if (!ix->implicit_ids) return;
+    ix->h_rowids.resize((size_t)ix->n);
+    for (long long i = 0; i < ix->n; ++i) ix->h_rowids[(size_t)i] = ix->first_seq + i + 1;
+    ix->implicit_ids = false;
+}
+
 // src_stride: bytes between rows in host memory; src_off: offset of the vector inside a row
 static int append_rows(vsb_index *ix, const uint8_t *src, size_t src_stride, size_t src_off, const int64_t *rowids,
                        bool ids_inline, int64_t nrows) {
@@ -961,36 +980,21 @@ static int append_rows(vsb_index *ix, const uint8_t *src, size_t src_stride, siz
     CU(cudaSetDevice(ix->device));
     const size_t rowbytes = (size_t)ix->dim * ix->esize;
     const size_t pitch = (size_t)ix->pitch;
-    const bool have_ids = ids_inline || rowids != nullptr;
-    if (have_ids && ix->implicit_ids) {
-        // materialise the implicit ids of rows appended so far
-        ix->h_rowids.resize((size_t)ix->n);
-        for (long long i = 0; i < ix->n; ++i) ix->h_rowids[(size_t)i] = ix->first_seq + i + 1;
-        ix->implicit_ids = false;
-    }
+    if (ids_inline || rowids != nullptr) materialise_ids(ix);
     if (pitch > kStageBuf) return fail(VSB_ERANGE, "row pitch %zu exceeds the %zu-byte staging buffer", pitch, (size_t)kStageBuf);
     const int64_t per_buf = (int64_t)(kStageBuf / pitch);
-    int64_t done = 0;
-    if (ix->streamed) {                      // the pinned arena IS the staging area
-        for (int64_t r = 0; r < nrows; ++r) {
-            const uint8_t *row = src + (size_t)r * src_stride;
-            uint8_t *dst = ix->h_arena + (size_t)(ix->n + r) * pitch;
-            memcpy(dst, row + src_off, rowbytes);
-            if (pitch > rowbytes) memset(dst + rowbytes, 0, pitch - rowbytes);
-            if (ids_inline) {
-                uint64_t v = 0;
-                for (int i = 7; i >= 0; --i) v = (v << 8) | row[i];
-                ix->h_rowids.push_back((int64_t)v);
-            }
+    for (int64_t done = 0; done < nrows;) {
+        // a streamed index takes all rows straight into its pinned arena; a resident one goes through the staging buffers
+        const int64_t m = ix->streamed ? nrows : std::min<int64_t>(per_buf, nrows - done);
+        int b = 0;
+        uint8_t *dst;
+        if (ix->streamed) {
+            dst = ix->h_arena + (size_t)ix->n * pitch;
+        } else {
+            const int rc = stage_acquire(ix, &b);
+            if (rc) return rc;
+            dst = ix->stage[b];
         }
-        done = nrows;
-    }
-    while (done < nrows) {
-        const int64_t m = std::min<int64_t>(per_buf, nrows - done);
-        int b;
-        int rc = stage_acquire(ix, &b);
-        if (rc) return rc;
-        uint8_t *dst = ix->stage[b];
         for (int64_t r = 0; r < m; ++r) {
             const uint8_t *row = src + (size_t)(done + r) * src_stride;
             memcpy(dst + (size_t)r * pitch, row + src_off, rowbytes);
@@ -1001,8 +1005,10 @@ static int append_rows(vsb_index *ix, const uint8_t *src, size_t src_stride, siz
                 ix->h_rowids.push_back((int64_t)v);
             }
         }
-        CU(cudaMemcpyAsync(ix->d_vec + (size_t)(ix->n + done) * pitch, dst, (size_t)m * pitch, cudaMemcpyHostToDevice, ix->stream));
-        CU(cudaEventRecord(ix->stage_ev[b], ix->stream));
+        if (!ix->streamed) {
+            CU(cudaMemcpyAsync(ix->d_vec + (size_t)(ix->n + done) * pitch, dst, (size_t)m * pitch, cudaMemcpyHostToDevice, ix->stream));
+            CU(cudaEventRecord(ix->stage_ev[b], ix->stream));
+        }
         done += m;
     }
     if (!ids_inline) {
@@ -1038,11 +1044,7 @@ int vsb_index_append_device(vsb_index *ix, const void *d_vectors, const int64_t 
     CU(cudaMemcpy2DAsync(ix->d_vec + (size_t)ix->n * ix->pitch, (size_t)ix->pitch, d_vectors, rowbytes, rowbytes, (size_t)nrows,
                          cudaMemcpyDeviceToDevice, ix->stream));
     if (d_rowids) {
-        if (ix->implicit_ids) {
-            ix->h_rowids.resize((size_t)ix->n);
-            for (long long i = 0; i < ix->n; ++i) ix->h_rowids[(size_t)i] = ix->first_seq + i + 1;
-            ix->implicit_ids = false;
-        }
+        materialise_ids(ix);
         ix->h_rowids.resize((size_t)(ix->n + nrows));
         CU(cudaMemcpyAsync(ix->h_rowids.data() + ix->n, d_rowids, sizeof(int64_t) * (size_t)nrows, cudaMemcpyDeviceToHost, ix->stream));
     } else if (!ix->implicit_ids) {
@@ -1101,16 +1103,8 @@ void vsb_index_free(vsb_index *ix) {
         if (ix->stage_ev[b]) cudaEventDestroy(ix->stage_ev[b]);
     }
     free_slots(ix);
-    for (int i = 0; i < kWorks; ++i) {
-        Work &w = ix->work[i];
-        for (int g = 0; g < kMaxGroup; ++g) {
-            if (w.q[g].d_lists) cudaFree(w.q[g].d_lists);
-            if (w.q[g].d_logs) cudaFree(w.q[g].d_logs);
-            if (w.q[g].d_counts) cudaFree(w.q[g].d_counts);
-            if (w.q[g].d_tlocal) cudaFree(w.q[g].d_tlocal);
-        }
-        if (w.d_bounds) cudaFree(w.d_bounds);
-        if (w.d_cta_time) cudaFree(w.d_cta_time);
+    free_workspaces(ix);
+    for (Work &w : ix->work) {
         if (w.scanned) cudaEventDestroy(w.scanned);
         if (w.drained) cudaEventDestroy(w.drained);
     }
@@ -1156,15 +1150,10 @@ int vsb_scan_topk(vsb_index *ix, int metric, const void *queries, int nq, int k,
         if (nq > 1) mi = 0;                      // batches: independent queries, like B separate cursors
         int rc = query_candidates(ix, metric, (const uint8_t *)queries + (size_t)b * qbytes, k, cands);
         if (rc) return rc;
-        SlotState s{k, mi, out_dist + (size_t)b * k, out_rowids + (size_t)b * k};
-        slots_begin(s);
-        for (const uint2 &c : cands) {
-            float d;
-            memcpy(&d, &c.x, 4);
-            slots_offer(s, d, rowid_of(ix, c.y));
-        }
+        SlotReplay s(k, mi, out_dist + (size_t)b * k, out_rowids + (size_t)b * k);
+        for (const uint2 &c : cands) s.offer_bits(c.x, rowid_of(ix, c.y));
         mi = s.mi;
-        const int cnt = slots_finish(s);
+        const int cnt = s.finish();
         if (out_counts) out_counts[b] = cnt;
     }
     if (max_index && nq == 1) *max_index = mi;
@@ -1174,13 +1163,8 @@ int vsb_scan_topk(vsb_index *ix, int metric, const void *queries, int nq, int k,
 int vsb_scan_all(vsb_index *ix, int metric, const void *query, float *out_dist, int64_t *out_rowids) {
     if (check_index(ix)) return VSB_EINVAL;
     if (!query || !out_dist) return fail(VSB_EINVAL, "bad scan arguments");
-    CU(cudaSetDevice(ix->device));
-    int rc = ensure_slots(ix);
-    if (rc) return rc;
-    rc = stage_query(ix, &ix->slot[0], query, ix->stream);
-    if (rc) return rc;
     std::vector<float> dist;
-    rc = scan_all_into(ix, metric, ix->slot[0].d_query, dist);
+    const int rc = query_all_distances(ix, metric, query, dist);
     if (rc) return rc;
     memcpy(out_dist, dist.data(), sizeof(float) * (size_t)ix->n);
     if (out_rowids)
@@ -1218,11 +1202,10 @@ int vsb_scan_candidates(vsb_index *ix, int metric, const void *queries, int nq, 
 int vsb_replay_topk(const vsb_candidate *cands, int n, int k, int *max_index, int64_t *out_rowids, double *out_dist) {
     if (k <= 0) return 0;
     if ((!cands && n > 0) || !out_rowids || !out_dist) return fail(VSB_EINVAL, "bad replay arguments");
-    SlotState s{k, max_index ? *max_index : 0, out_dist, out_rowids};
-    slots_begin(s);
-    for (int i = 0; i < n; ++i) slots_offer(s, cands[i].dist, cands[i].rowid);
+    SlotReplay s(k, max_index ? *max_index : 0, out_dist, out_rowids);
+    for (int i = 0; i < n; ++i) s.offer(cands[i].dist, cands[i].rowid);
     if (max_index) *max_index = s.mi;
-    return slots_finish(s);
+    return s.finish();
 }
 
 int vsb_debug_read(vsb_index *ix, const char *name, void *out, int64_t bytes) {
@@ -1273,28 +1256,10 @@ int vsb_profile_read(vsb_index *ix, double *scan_ms, int *scan_launches, double 
 int vsb_scan_submit(vsb_index *ix, int metric, const void *query, int query_on_device, int k, int fetch, int want_slot) {
     if (check_index(ix)) return VSB_EINVAL;
     if (!query || k <= 0 || k > kMaxK) return fail(VSB_EINVAL, "bad scan arguments (k must be 1..%d)", kMaxK);
-    CU(cudaSetDevice(ix->device));
-    int rc = ensure_slots(ix);
-    if (rc) return rc;
-    rc = ensure_workspace(ix, k);
-    if (rc) return rc;
     if (want_slot >= kSlots) return fail(VSB_EINVAL, "slot %d out of range (have %d)", want_slot, kSlots);
     const int si = want_slot >= 0 ? want_slot : (ix->last_slot + 1) % kSlots;
-    Slot *slot = &ix->slot[si];
-    const uint8_t *dq = (const uint8_t *)query;
-    cudaStream_t ss = next_scan_stream(ix);
-    if (!query_on_device) {
-        // the slot's pinned staging buffer is free once the slot's previous query has completed on the device
-        if (slot->seq > 0) CU(cudaEventSynchronize(slot->done));
-        rc = stage_query(ix, slot, query, ss);
-        if (rc) return rc;
-        dq = slot->d_query;
-    }
-    rc = launch_scan(ix, metric, dq, k, slot, nullptr, fetch != 0, ss);
-    if (rc) return rc;
-    ix->last_slot = si;
-    ix->last_metric = metric;
-    return si;   // slot id (>= 0) for vsb_collect / vsb_result_block
+    const int rc = submit_group(ix, metric, query, 0, 1, query_on_device, k, fetch, si, false);
+    return rc ? rc : si;   // slot id (>= 0) for vsb_collect / vsb_result_block
 }
 
 int vsb_scan_submit_group(vsb_index *ix, int metric, const void *queries, int64_t query_stride, int nq, int query_on_device, int k,
@@ -1391,14 +1356,9 @@ int vsb_collect(vsb_index *ix, int slot_id, int k, int64_t *out_rowids, double *
     int n = gather_survivors(ix, &ix->slot[slot_id], cands, &overflow);
     if (n < 0) return n;
     if (overflow) return fail(VSB_ERANGE, "candidate log overflowed; use vsb_scan_topk (host query) for this input");
-    SlotState s{k, 0, out_dist, out_rowids};
-    slots_begin(s);
-    for (const uint2 &c : cands) {
-        float d;
-        memcpy(&d, &c.x, 4);
-        slots_offer(s, d, rowid_of(ix, c.y));
-    }
-    const int cnt = slots_finish(s);
+    SlotReplay s(k, 0, out_dist, out_rowids);
+    for (const uint2 &c : cands) s.offer_bits(c.x, rowid_of(ix, c.y));
+    const int cnt = s.finish();
     if (out_count) *out_count = cnt;
     return VSB_OK;
 }

@@ -645,6 +645,24 @@ __global__ void __launch_bounds__(kThreads, 1) scan_kernel(const ScanParams prm)
 // bound.  We use  min( k-th smallest over all streams of earlier segments,
 //                      k-th smallest over the earlier streams of the same segment ),
 // both built from the streams' final k-lists (each contains the k smallest values of its stream).
+//
+// Result head of one query, written by filter_kernel and read by the host and by the peers of an exchange:
+//   [header: ints kHdr*, kHdrBytes][block table: (first survivor, count) per filter block, kTableCap x int2][survivors]
+// Survivors are (distance bits, local row) in scan order once taken block by block through the table; the first
+// header[kHdrHeadcap] of them sit in the head, the rest in a separate tail.
+constexpr int kHdrTotal = 0;      // survivors of the query
+constexpr int kHdrFlags = 1;      // 0, or kHdrOverflow / kHdrLost
+constexpr int kHdrSeq = 2;        // launch sequence number of the result slot
+constexpr int kHdrBlocks = 3;     // filter blocks: used entries of the block table
+constexpr int kHdrXseq = 4;       // exchange sequence number
+constexpr int kHdrSrc = 5;        // shard that produced the head
+constexpr int kHdrHeadcap = 6;    // survivors carried in the head itself
+constexpr int kHdrOverflow = 1;   // flag: the candidate log or the survivor capacity overflowed
+constexpr int kHdrLost = 8;       // flag: the receiving side stopped waiting for this head (peer lost)
+constexpr int kHdrBytes = 64;     // offset of the block table
+constexpr int kTableCap = 512;
+constexpr size_t kResHdrBytes = kHdrBytes + sizeof(int2) * kTableCap;   // offset of the survivors
+
 struct FilterQuery {    // per-query pointers of a (group) launch: blockIdx.y selects the query
     const float *lists; // k <= 32: [S / kWarps][32] sorted CTA lists; else [S][kcap] stream lists
     const float *tlocal;// k <= 32: [S] in-CTA prefix bound of each stream (from scan_kernel)
@@ -653,11 +671,11 @@ struct FilterQuery {    // per-query pointers of a (group) launch: blockIdx.y se
     uint2 *out;         // survivors (dist bits, local row), grouped by block in stream order: the first headcap of them
     uint2 *out_tail;    //   go to out (inside the slot's head, the part that travels), the rest to out_tail
     int2 *table;        // [gridDim.x] (base, count) of each block's survivors in out
-    int *hdr;           // hdr[0] = total survivors, hdr[1] = overflow flag, hdr[2] = sequence number
+    int *hdr;           // the result header (kHdr* fields)
     int *ctrl;          // device: [0] cursor, [1] overflow from scan_kernel, [2] blocks done
     int seqno;
     int xslot;          // push: slot row of the targets' gather buffers
-    unsigned xseq;      // push: exchange sequence number published with the head (hdr[4]) and raised on the flags
+    unsigned xseq;      // push: exchange sequence number published with the head (kHdrXseq) and raised on the flags
 };
 
 // NVLink peer-memory all-gather, fused into the filter: the block that completes a query's result head copies the used part
@@ -670,7 +688,7 @@ struct PushParams {
     int ntargets;                 // 0: nothing is pushed (single shard)
     int src;                      // this shard's index inside a slot's gather row
     int world;                    // shards per slot in the gather layout [slots][world][head_bytes]
-    int head_bytes, res_hdr_bytes;// layout of a head: [hdr 64 B][table][survivors from res_hdr_bytes on]
+    int head_bytes, res_hdr_bytes;// layout of a head: [header][table][survivors from res_hdr_bytes on]
     int tailcap;                  // survivors beyond the head's headcap travel to a separate tail row of this many entries
     uint8_t *gather[kMaxPeers];   // target t: base of its gather buffer
     unsigned *flags[kMaxPeers];   // target t: [slots][world] arrival flags (the exchange sequence number of the slot)
@@ -687,7 +705,7 @@ __device__ __forceinline__ unsigned ld_acquire_sys(const unsigned *p) {
 }
 
 // receiving side: one thread per (slot of the group, source shard) spins until that shard's flag carries the expected
-// sequence number.  Bounded: after `timeout` clock cycles the missing head is marked (hdr[1] |= 8) so that the merge reports
+// sequence number.  Bounded: after `timeout` clock cycles the missing head is marked (kHdrLost) so that the merge reports
 // an error instead of the GPU hanging on a peer that died.
 struct WaitParams {
     const unsigned *flags;        // [slots][world]
@@ -704,7 +722,7 @@ __global__ void exchange_wait_kernel(const WaitParams wp) {
     const long long t0 = clock64();
     while (ld_acquire_sys(wp.flags + at) != wp.xseq[j]) {
         if (clock64() - t0 > wp.timeout) {
-            reinterpret_cast<int *>(wp.gather + at * wp.head_bytes)[1] = 8;
+            reinterpret_cast<int *>(wp.gather + at * wp.head_bytes)[kHdrFlags] = kHdrLost;
             break;
         }
         __nanosleep(200);
@@ -717,8 +735,8 @@ __global__ void exchange_wait_kernel(const WaitParams wp) {
 // stream order after the filters).
 __device__ __forceinline__ void push_one_head(const PushParams &pp, const int *hdr, const uint2 *out, const uint2 *out_tail, int xslot, unsigned xseq,
                                               int headcap) {
-    const int total = max(__ldcg(hdr), 0), nblocks = __ldcg(hdr + 3);
-    const int nhead = 8 + nblocks;                                         // uint2 words of header + block table
+    const int total = max(__ldcg(hdr + kHdrTotal), 0), nblocks = __ldcg(hdr + kHdrBlocks);
+    const int nhead = kHdrBytes / (int)sizeof(uint2) + nblocks;            // uint2 words of header + block table
     const int nsurv = min(total, headcap);
     const int ntail = min(max(total - headcap, 0), pp.tailcap);
     const uint2 *src_head = reinterpret_cast<const uint2 *>(hdr);
@@ -995,13 +1013,13 @@ __global__ void __launch_bounds__(filter_warps(FAST) * 32, 1) filter_kernel(cons
             __threadfence();
             const int total = atomicAdd(&fq.ctrl[0], 0);
             const int ovf = atomicAdd(&fq.ctrl[1], 0);
-            fq.hdr[0] = total;
-            fq.hdr[1] = (ovf != 0 || total > fp.outcap) ? 1 : 0;
-            fq.hdr[2] = fq.seqno;
-            fq.hdr[3] = (int)gridDim.x;
-            fq.hdr[4] = (int)fq.xseq;
-            fq.hdr[5] = fp.push.src;
-            fq.hdr[6] = fp.headcap;
+            fq.hdr[kHdrTotal] = total;
+            fq.hdr[kHdrFlags] = (ovf != 0 || total > fp.outcap) ? kHdrOverflow : 0;
+            fq.hdr[kHdrSeq] = fq.seqno;
+            fq.hdr[kHdrBlocks] = (int)gridDim.x;
+            fq.hdr[kHdrXseq] = (int)fq.xseq;
+            fq.hdr[kHdrSrc] = fp.push.src;
+            fq.hdr[kHdrHeadcap] = fp.headcap;
             fq.ctrl[0] = 0; fq.ctrl[1] = 0; fq.ctrl[2] = 0;
         }
         is_last = last;
